@@ -193,8 +193,11 @@ def run_ours(args):
     barrier(dist, local)
     ctx.timer_start()
     for _ in range(K):
-        step()
+        last = step()
     ms = ctx.timer_stop()
+    if args.dump_outputs and rank == 0:
+        eig_last, sum_last = f.read_back()          # the factor cache the last step left behind (read before any later step overwrites it)
+        dump_outputs(args.dump_outputs, last, eig_last, sum_last)
     ms = barrier_max(dist, local, ms)
     clocks = sampler.stop()
     launches = ctx.launches - launches0
@@ -346,6 +349,34 @@ def run_ours(args):
         print(json.dumps(line), flush=True)
     if dist is not None:
         dist.barrier(); dist.destroy_process_group()
+
+
+DUMP_CAP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, o, eig12, sum10, cap=DUMP_CAP_BYTES):
+    """What the last timed step returned to its caller, as DIR/<name>.npy (float64): the LI-BA states, the residual pair, the LM trace
+    (r1, r2, u, v, q1, accepted, hess_built per iteration) and the factor cache the step leaves behind (eig12 / sum10 per voxel, what the
+    reference's LidarFactor holds after damping_iter).  Inputs are seeded, so two builds run with the same arguments can be compared file by file;
+    the fp64 atomic sums make even two runs of one build differ in the last bits (relative ~1e-9 on the smallest eigenvalues of eig12).
+    Above `cap` bytes in all, the per-voxel arrays are replaced by the same fixed, seeded sample of voxels, whose indices go to voxel_index.npy."""
+    tr = o["trace"]
+    arrays = {"states": o["states"], "resis": o["resis"],
+              "trace": np.stack([tr[k].astype(np.float64) for k in ("r1", "r2", "u", "v", "q1", "accepted", "hess_built")], axis=1).reshape(-1, 7)}
+    per_voxel = {"factor_eig12": eig12, "factor_sum10": sum10}
+    fixed = sum(a.nbytes for a in arrays.values())
+    row_bytes = sum(a[0].nbytes for a in per_voxel.values())
+    V = len(eig12)
+    if fixed + V * row_bytes > cap:
+        keep = max(0, (cap - fixed - 4096) // (row_bytes + 8))   # + 8 B per voxel for voxel_index.npy, 4 KB for the .npy headers
+        sel = np.sort(np.random.default_rng(0).choice(V, keep, replace=False))
+        per_voxel = {k: a[sel] for k, a in per_voxel.items()}
+        arrays["voxel_index"] = sel.astype(np.float64)
+    arrays.update(per_voxel)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a, dtype=np.float64))
+    log(f"[dump] {len(arrays)} arrays, {sum(a.nbytes for a in arrays.values())} bytes -> {out_dir}")
 
 
 def parity_block(vx, ctx, W, ptr, fr, cl, eig, s, est, first_step, cpu):
@@ -720,6 +751,8 @@ def cpu_baseline_from_structure(vx, W, ptr, fr, cl, eig, s, st0, tr, reps=2):
             out["reference_sources"] = {"value": 1.0 / min(tr_), "unit": UNIT, "cores": 5, "kind": "reference", "iterations_per_call": iters,
                                         "sample": "the reference's LI_BA_Optimizer::damping_iter (voxel_map.hpp compiled unmodified against the stand-in Eigen: scalar loops, no SSE packet "
                                                   "math; real IMU_PRE objects) on the same factor, best of 2 calls, call time / iterations executed"}
+        else:
+            out["reference_sources"] = {"unavailable": "oracle/_ref/libvxref.so was not built (it needs the original project's sources at build time)"}
     except Exception as e:          # noqa: BLE001 — the extra figure must never cost the bench line
         out["reference_sources"] = {"error": repr(e)}
     return out
@@ -982,7 +1015,12 @@ def main():
     ap.add_argument("--gba-pts", type=int, default=50000)
     ap.add_argument("--gba-per-row", type=int, default=20)
     ap.add_argument("--gba-voxel", type=float, default=1.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy (default local-BA workload of --impl ours)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.workload != "local_ba" or args.impl != "ours"):
+        ap.error("--dump-outputs applies to the default local_ba workload of --impl ours")
     if args.workload == "hba":     # the hierarchical global-BA leg alone (same JSON block as the `gba` key of the default run)
         import voxel_slam_b200 as vx
         rank, world, local, dist = dist_setup(args)

@@ -110,24 +110,6 @@ def test_cpp_shim_typed_layer_type_checks_against_reference_signatures():
 
 
 
-def test_cpp_shim_typed_layer_compiles_against_the_reference_headers():
-    """The typed layer against the reference's REAL tools.hpp / preintegration.hpp / voxel_map.hpp (IMUST, PointCluster, IMU_PRE, pointVar,
-    SlideWindow, Keyframe, PLV ...), with the stand-in Eigen / PCL / ROS headers of oracle/ref_standin; skipped where /root/reference is absent
-    (the stub-based check above still runs there).  Also checks the layout assumptions (sizeof(pointVar), sizeof(PointType))."""
-    import subprocess
-    import tempfile
-    import pytest
-    ref = "/root/reference/VoxelSLAM/src"
-    if not os.path.exists(os.path.join(ref, "voxel_map.hpp")):
-        pytest.skip("reference sources not present on this box")
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    src = '#include "voxel_map.hpp"\nstatic_assert(sizeof(pointVar) == 96 && sizeof(PointType) == 48, "record layouts the C-ABI relies on");\n' + SHIM_USE
-    with tempfile.NamedTemporaryFile("w", suffix=".cpp", delete=False) as f:
-        f.write(src)
-    r = subprocess.run(["g++", "-std=c++17", "-fsyntax-only", "-w", "-I", os.path.join(root, "oracle", "ref_standin"), "-I", ref, "-I", root, f.name], capture_output=True, text=True)
-    assert r.returncode == 0, r.stderr[-4000:]
-
-
 def test_bench_reference_arm_contract_on_cpu():
     """`bench.py --impl reference` needs no GPU: one JSON line with the contract keys (tiny window so that it runs in seconds)."""
     import json
